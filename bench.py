@@ -126,7 +126,7 @@ def nbytes(data):
 # ------------------------------------------------------------------------------------------------
 class CpuArm:
     """The reference's own implementation of the path on the host CPU cores (BASELINE.md section 4): the UNMODIFIED
-    reference matcher driven through its real TwoViewPipeline (oracle/reference_runner.py; installed under baseline/_ref
+    reference matcher driven through its real TwoViewPipeline (oracle/reference_runner.py; installed under oracle/_ref
     by the build, `kind: "reference"`), or, when that copy did not travel, the oracle port (`kind: "port"`).
     One step = zero_grad + forward + loss + backward + Adam on `B` pairs of the N=2048 / 9-layer workload, fp32."""
 
@@ -249,7 +249,7 @@ def gpu_eager_baseline(dev, B=4, steps=5, warmup=3):
     from oracle import reference_runner as R
 
     if not R.available():
-        return {"unavailable": "baseline/_ref did not travel (reference not installed)"}
+        return {"unavailable": "reference not installed under oracle/_ref"}
     conf = dict(synthetic.DEFAULT_CONF)
     w = synthetic.make_weights(conf, seed=0)
     batch = synthetic.to_device(R.pipeline_batch(synthetic.make_pairs(B, N_KPTS, seed=1234)), dev)
@@ -292,6 +292,8 @@ def main():
     ap.add_argument("--no-kernel-timing", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from the host instead of replaying "
                     "one CUDA graph of the whole training step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed "
+                    "(loss, per-pair loss terms, updated parameters) as DIR/<name>.npy, so that two builds can be compared")
     args = ap.parse_args()
 
     global N_KPTS, ATTN_FLOPS_PER_PAIR
@@ -357,11 +359,15 @@ def main():
     if use_graph:
         trainer.capture(pool_dev[0], dev, warmup=2)
 
+    last = []  # (loss, losses) of the latest resident step
+
     def step_resident(i):
         if use_graph:
-            trainer.step_graphed(pool_dev[i % len(pool_dev)])  # device-to-device copy into the static inputs + replay
+            last[:] = trainer.step_graphed(pool_dev[i % len(pool_dev)])  # device-to-device copy into the static inputs + replay
         else:
-            trainer.step(pool_dev[i % len(pool_dev)])
+            loss, losses = trainer.step(pool_dev[i % len(pool_dev)])
+            # detached: holding the loss terms must not keep the step's autograd graph alive into the next step
+            last[:] = loss, {k: v.detach() if torch.is_tensor(v) else v for k, v in losses.items()}
 
     host_loss = []
 
@@ -380,6 +386,8 @@ def main():
         ms = timed(step_resident, args.steps)
         launches = launches_per_step * args.steps
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last, model)
     # dominant kernel, timed live with CUDA events on the launching stream (second pass, so the
     # event records do not perturb the headline number)
     roof = None
@@ -424,6 +432,21 @@ def main():
         dist.barrier()
         sys.stdout.flush()
         os._exit(0)
+
+
+def dump_outputs(out_dir, loss, losses, model):
+    """What a caller of the timed training step receives from its last call: the mean loss, every per-pair loss term and
+    the parameters the optimiser step updated in place (all of them: 47.4 MB in float32 at d=256, L=9).  The inputs are
+    seeded, so the same arguments give the same files up to floating-point reordering."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss}
+    arrays.update({f"losses.{k}": v for k, v in losses.items() if torch.is_tensor(v)})
+    arrays.update({f"param.{k}": p for k, p in model.named_parameters()})
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy() if t.dtype == torch.float64 else t.float().numpy())
 
 
 def kernel_roofline(trainer, pool_dev, B, dev):

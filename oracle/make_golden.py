@@ -83,9 +83,6 @@ def run_case(name, conf, B, N, M, seed, dtype=torch.float64, sub=1):
     out["pred|log_assignment"] = la[:, ::sub, ::sub].cpu().numpy()
     out["pred|log_assignment_rowmax"] = la[:, :-1, :-1].max(2).values.cpu().numpy()
     out["pred|log_assignment_colmax"] = la[:, :-1, :-1].max(1).values.cpu().numpy()
-    rd0 = pred["ref_descriptors0"].detach()
-    out["pred|ref_descriptors0_sub"] = rd0[:, :, :: max(1, N // 16)].cpu().numpy()
-    out["pred|ref_descriptors1_sub"] = pred["ref_descriptors1"].detach()[:, :, :: max(1, N // 16)].cpu().numpy()
     for k, v in losses.items():
         out["loss|" + k] = v.detach().cpu().numpy() if torch.is_tensor(v) else np.array(v)
     for k, p in model.named_parameters():
@@ -217,9 +214,9 @@ def run_gluestick_attention():
     w = torch.from_numpy(rs.standard_normal((b, d, h, n)))
     o, _ = attention(q, k, v)
     (o * w).sum().backward()
-    out.update({"core|q": q.detach().numpy(), "core|k": k.detach().numpy(), "core|v": v.detach().numpy(),
-                "core|w": w.numpy(), "core|out": o.detach().numpy(), "core|dq": q.grad.numpy(),
-                "core|dk": k.grad.numpy(), "core|dv": v.grad.numpy()})
+    # the inputs q, k, v, w (and x, src, w2 below) are not stored: tests re-draw them from RandomState(21)
+    out.update({"core|out": o.detach().numpy(), "core|dq": q.grad.numpy(), "core|dk": k.grad.numpy(),
+                "core|dv": v.grad.numpy()})
     # module level: weights drawn from the seeded stream below (the test rebuilds them), gradients summarised
     b, n, m = 1, 40, 56
     mha = MultiHeadedAttention(4, 256).double()
@@ -232,8 +229,7 @@ def run_gluestick_attention():
     w2 = torch.from_numpy(rs.standard_normal((b, 256, n)))
     y = mha(x, src, src)
     (y * w2).sum().backward()
-    out.update({"mha|x": x.detach().numpy(), "mha|src": src.detach().numpy(), "mha|w": w2.numpy(),
-                "mha|out": y.detach().numpy(), "mha|dx": x.grad.numpy(), "mha|dsrc": src.grad.numpy(),
+    out.update({"mha|out": y.detach().numpy(), "mha|dx": x.grad.numpy(), "mha|dsrc": src.grad.numpy(),
                 "mha|param_names": np.array([n_ for n_, _ in mha.named_parameters()])})
     for name, p_ in mha.named_parameters():
         out.update(summarise("mha|grad|" + name, p_.grad))
@@ -393,6 +389,26 @@ def run_eval_loss():
     print("eval_loss ->", path, {k: v for k, v in out.items() if k.startswith("loss|total")})
 
 
+def run_dropin_surface():
+    """What a drop-in replacement of the reference's LightGlue matcher and homography ground-truth component must
+    reproduce (models/matchers/lightglue.py, models/matchers/homography_matcher.py): the matcher's state_dict names,
+    shapes and confidence thresholds at n_layers=2, and the ground-truth component's default_conf and
+    required_data_keys."""
+    from gluefactory.models import get_model
+
+    lg = get_model("matchers.lightglue")({"n_layers": 2})
+    gt = get_model("matchers.homography_matcher")
+    out = {"lightglue|keys": np.array(list(lg.state_dict().keys())),
+           "lightglue|confidence_thresholds": lg.confidence_thresholds.numpy(),
+           "homography|required_data_keys": np.array(sorted(gt({}).required_data_keys)),
+           "homography|default_conf": np.array(repr(dict(gt.default_conf)))}
+    for k, v in lg.state_dict().items():
+        out["lightglue|shape|" + k] = np.array(tuple(v.shape), dtype=np.int64)
+    path = os.path.join(OUT, "dropin_surface.npz")
+    np.savez_compressed(path, **out)
+    print("dropin_surface ->", path)
+
+
 def run_autocast_cases():
     torch.manual_seed(0)
     mid = dict(synthetic.DEFAULT_CONF, n_layers=3, filter_threshold=0.1)
@@ -409,6 +425,7 @@ if __name__ == "__main__":
         for name in only:
             {"gluestick_attn": run_gluestick_attention, "gt_homography": run_gt_homography,
              "heads_grad": run_heads_grad, "autocast": run_autocast_cases, "eval_loss": run_eval_loss, "gluestick": run_gluestick, "gt_pose_depth": run_gt_pose_depth, "adaptive": run_adaptive,
+             "dropin": run_dropin_surface,
              "sift": lambda: run_case("lg_sift_d256_l2_n96", dict(synthetic.DEFAULT_CONF, n_layers=2, input_dim=128,
                                                                   add_scale_ori=True), B=1, N=96, M=80, seed=16)}[name]()
         sys.exit(0)
@@ -433,3 +450,4 @@ if __name__ == "__main__":
     run_gluestick()
     run_gt_pose_depth()
     run_adaptive()
+    run_dropin_surface()

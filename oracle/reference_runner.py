@@ -1,4 +1,4 @@
-"""Drive the UNMODIFIED reference (installed under baseline/_ref by oracle/stage_reference.py) through its own public
+"""Drive the UNMODIFIED reference (installed under oracle/_ref by oracle/stage_reference.py) through its own public
 API for the hot path: `TwoViewPipeline` with `extractor.name = None`, features supplied through `view*["cache"]`
 (the cached-feature route, two_view_pipeline.py:62-70), `matcher.name = matchers.lightglue`, and the body of the
 training loop restated from train.py:456-517 (zero_grad -> autocast(forward, loss) -> mean -> scaled backward ->
@@ -17,7 +17,7 @@ def available():
 def build_pipeline(conf, weights, device="cpu", checkpointed=False, flash=False):
     """conf: LightGlue conf (synthetic.DEFAULT_CONF keys); weights: state_dict under the reference names."""
     get_model = import_reference()
-    assert get_model is not None, "reference not installed under baseline/_ref (run oracle/stage_reference.py)"
+    assert get_model is not None, "reference not installed under oracle/_ref (run oracle/stage_reference.py)"
     matcher_conf = {k: v for k, v in conf.items() if k not in ("precision", "engine", "stack_ref_descriptors")}
     matcher_conf.update(name="matchers.lightglue", checkpointed=bool(checkpointed), flash=bool(flash))
     pipe = get_model("two_view_pipeline")({

@@ -1,20 +1,18 @@
-"""Install the UNMODIFIED reference into baseline/_ref/ (TEST / BASELINE INFRASTRUCTURE ONLY -- the product package
-never imports it) and put it on sys.path for the reference arm of bench.py.
+"""Install the UNMODIFIED reference into oracle/_ref/ (TEST / BASELINE INFRASTRUCTURE ONLY -- the product package
+never imports it) and put it on sys.path for the reference arms of bench.py.
 
-/root/reference exists only in the build container; the GPU box sees what travels with the repo snapshot.
-baseline/_ref/ is git-ignored (no reference source ever enters the history) but NOT gpurun-ignored, so the installed
-package travels like the built .so.  The recipe is the one offline install the task statement allows:
+The reference tree is found at $GLUEFACTORY_REFERENCE.  oracle/_ref/ is git-ignored (no reference source ever enters
+the history); a machine without the reference tree simply has no oracle/_ref/.  The recipe is an offline install:
 
-    python -m pip install --no-index --no-build-isolation --no-deps --find-links /opt/wheelhouse \
-        --target baseline/_ref <copy of /root/reference under /tmp>
+    python -m pip install --no-index --no-build-isolation --no-deps --target oracle/_ref <copy of the reference tree>
 
-(--no-deps: omegaconf / kornia / h5py ... are not in the wheelhouse; the matcher's import closure -- 13 pure-Python
-files -- needs only torch, numpy and omegaconf, and omegaconf is covered by the ~100-line stand-in oracle/_shim/omegaconf;
-the copy under /tmp is needed because the wheel build writes into the source tree and /root/reference is read-only).
+(--no-deps: the matcher's import closure -- 13 pure-Python files -- needs only torch, numpy and omegaconf, and
+omegaconf is covered by the ~100-line stand-in oracle/_shim/omegaconf; the copy into a temporary directory is needed
+because the wheel build writes into the source tree, which may be read-only).
 
 `bench.py --impl reference` and its `gpu_eager_baseline` leg then time the reference's own modules
-(`cpu_baseline.kind = "reference"`); when baseline/_ref is absent they fall back to the oracle port (`"port"`).
-Run by __graft_entry__.build() whenever /root/reference is present.
+(`cpu_baseline.kind = "reference"`); when oracle/_ref is absent they fall back to the oracle port (`"port"`).
+Run by __graft_entry__.build() whenever the reference tree is present.
 """
 import os
 import shutil
@@ -23,9 +21,8 @@ import sys
 import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 REF = os.environ.get("GLUEFACTORY_REFERENCE", "/root/reference")
-DST = os.path.join(ROOT, "baseline", "_ref")
+DST = os.path.join(HERE, "_ref")
 
 
 def installed():
@@ -33,25 +30,25 @@ def installed():
 
 
 def stage(verbose=True, force=False):
-    """Returns True when baseline/_ref holds the installed reference."""
+    """Returns True when oracle/_ref holds the installed reference."""
     if installed() and not force:
         return True
     if not os.path.isdir(REF):
         if verbose:
-            print(f"[stage_reference] {REF} not present and baseline/_ref empty: reference arm falls back to the port")
+            print(f"[stage_reference] {REF} not present and oracle/_ref empty: reference arm falls back to the port")
         return False
     tmp = tempfile.mkdtemp(prefix="gf_ref_")
     try:
         src = os.path.join(tmp, "reference")
         shutil.copytree(REF, src, symlinks=True, ignore=shutil.ignore_patterns(".git"))
         os.makedirs(DST, exist_ok=True)
-        cmd = [sys.executable, "-m", "pip", "install", "--no-index", "--no-build-isolation", "--no-deps", "--find-links",
-               "/opt/wheelhouse", "--upgrade", "--target", DST, src]
+        cmd = [sys.executable, "-m", "pip", "install", "--no-index", "--disable-pip-version-check", "--no-build-isolation",
+               "--no-deps", "--upgrade", "--target", DST, src]
         r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
         if verbose or r.returncode:
             print(r.stdout[-800:])
         if r.returncode:
-            raise RuntimeError("pip install of the reference into baseline/_ref failed")
+            raise RuntimeError("pip install of the reference into oracle/_ref failed")
     finally:
         shutil.rmtree(tmp, ignore_errors=True)
     return installed()

@@ -1,5 +1,5 @@
 """GlueStick (points + lines, BASELINE configs[4]) training step on one B200: the plugin (bf16 and fp32) against the
-unmodified reference module from baseline/_ref in PyTorch eager on the same GPU (fp32 and bf16 autocast).
+unmodified reference module from oracle/_ref in PyTorch eager on the same GPU (fp32 and bf16 autocast).
 Forward + loss + backward + Adam, synthetic batch, N points and L lines per image."""
 import os
 import sys

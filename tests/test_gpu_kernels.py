@@ -14,7 +14,7 @@ import torch
 
 from gluefactory_b200 import ops
 from oracle import lightglue_oracle as O
-from tests.util import GOLDEN, rel_err
+from tests.util import GOLDEN, load_gluestick_attn, rel_err
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -515,7 +515,7 @@ def test_gt_from_homography_degenerate_rows():
 def test_gluestick_attention_matches_golden(dtype, tol):
     """SURVEY 8a row a15: GlueStick's channels-first attention core (gluestick.py:524-529), forward and gradients,
     against vectors produced by the reference function itself (oracle/make_golden.py)."""
-    g = dict(np.load(os.path.join(GOLDEN, "gluestick_attn.npz")))
+    g = load_gluestick_attn()
     q, k, v = (torch.from_numpy(g[f"core|{n}"]).to(dtype).to(DEV).requires_grad_() for n in "qkv")
     out = ops.gluestick_attention(q, k, v)
     assert out.shape == q.shape

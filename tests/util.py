@@ -25,6 +25,18 @@ def load_case(name, dtype=torch.float64):
     return g, conf, weights, data
 
 
+def load_gluestick_attn():
+    """tests/golden/gluestick_attn.npz with its inputs: the fixture stores the reference's outputs and gradients, the
+    inputs are re-drawn from the generator's seeded stream (oracle/make_golden.py run_gluestick_attention)."""
+    g = dict(np.load(os.path.join(GOLDEN, "gluestick_attn.npz"), allow_pickle=False))
+    rs = np.random.RandomState(21)
+    b, d, h, n, m = 1, 64, 4, 40, 56
+    for k, shape in (("core|q", (b, d, h, n)), ("core|k", (b, d, h, m)), ("core|v", (b, d, h, m)),
+                     ("core|w", (b, d, h, n)), ("mha|x", (b, 256, n)), ("mha|src", (b, 256, m)), ("mha|w", (b, 256, n))):
+        g[k] = rs.standard_normal(shape)
+    return g
+
+
 def probe_index(n, k=512):
     return torch.from_numpy(np.random.RandomState(n % 65521).randint(0, n, size=k))
 
